@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload perceive|lift_splat] [--batch b_per_gpu]
   python bench.py --impl reference ...     # the reference's CPU path (oracle port) on the host cores
+  python bench.py ... --dump-outputs DIR   # also write the last timed step's outputs as DIR/<name>.npy
 
 One "step" = one pass of the hot path over one batch of synthetic samples (6 cameras x 3 frames, 200x200 BEV);
 one "frame" of the metric = one sample's BEV perception output.  Rank 0 prints ONE JSON line.
@@ -141,6 +142,30 @@ def make_problem(cfg, batch, seed, tilt_deg=0.0):
                 off=G.bev_offset(start, res))
 
 
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(outputs, directory, limit=DUMP_LIMIT_BYTES):
+    """--dump-outputs: every tensor of `outputs` (what the timed step returned) as <directory>/<name>.npy, float64 kept,
+    anything else as float32.  When together they exceed `limit` bytes, each file holds a fixed sample of its array's
+    flattened entries instead (indices drawn with seed 0 and sorted: the same for the same shapes in every run), sized
+    so that all files fit.  Inputs are seeded, so two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    arrays = {}
+    for name, t in outputs.items():
+        if isinstance(t, torch.Tensor):
+            t = t.detach()
+            arrays[name] = (t if t.dtype == torch.float64 else t.float()).cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    budget = limit - 1024 * len(arrays)          # room for the .npy headers
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        if total > limit:
+            keep = max(1, a.size * budget // total)
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
 def build_model(device=None, lcfg=None):
     """Random-init (seeded, machine-independent) perception model; the trunk is not needed (inputs enter after it)."""
     from stp3_b200.config import get_cfg
@@ -175,8 +200,8 @@ def workload_config(args, cfg, world):
 
 class ReferenceArm:
     """The reference's own CPU implementation of the path on the host cores.  kind "reference": the UNMODIFIED
-    reference package (installed by oracle/build_ref.py into the git-ignored baseline/_ref/, or /root/reference in the
-    build container) -- its STP3.get_geometry / projection_to_birds_eye_view, TemporalModel and Decoder -- imported
+    reference package (installed by oracle/build_ref.py into the git-ignored oracle/_ref/, or the checkout named by
+    STP3_REFERENCE_ROOT) -- its STP3.get_geometry / projection_to_birds_eye_view, TemporalModel and Decoder -- imported
     through oracle/ref_loader.py; kind "port": the op-for-op CPU port under oracle/ when that install is absent."""
 
     def __init__(self, workload, cfg):
@@ -255,14 +280,14 @@ class ReferenceArm:
         times = []
         for _ in range(steps):
             t0 = time.perf_counter()
-            self.step()
+            self.last = self.step()
             times.append(time.perf_counter() - t0)
         dt = statistics.median(times)
         return {"fps": 1.0 / dt, "dt": dt, "threads": threads, "times": times,
                 "sweep": {str(k): round(v, 3) for k, v in sweep.items()}}
 
     def describe(self, r, steps, warmup):
-        what = ("unmodified reference package (baseline/_ref or /root/reference via oracle/ref_loader.py): STP3.get_geometry + "
+        what = ("unmodified reference package (oracle/_ref or STP3_REFERENCE_ROOT via oracle/ref_loader.py): STP3.get_geometry + "
                 "projection_to_birds_eye_view" + (" + TemporalModel + Decoder" if self.workload in PERCEPTION else "")
                 if self.kind == "reference" else
                 "op-for-op CPU port of the reference (oracle/torch_port.py" + (" + oracle/torch_dense.py)" if self.workload in PERCEPTION else ")"))
@@ -286,6 +311,8 @@ def run_reference_arm(args, cfg):
                          "sample": arm.describe(r, steps, warmup)},
         "e2e": {"value": r["fps"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
+    if args.dump_outputs:
+        dump_outputs(arm.last if isinstance(arm.last, dict) else {"bev": arm.last}, args.dump_outputs)
     print(json.dumps(line), flush=True)
 
 
@@ -368,7 +395,12 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the sustained run, the second rig and the latency mode")
     ap.add_argument("--profiler-range", action="store_true",
                     help="bracket the resident timed steps with cudaProfilerStart/Stop (ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (rank 0's shard; "
+                         f"at most {DUMP_LIMIT_BYTES // 10**6} MB in all, a fixed seeded sample of each output beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = syn.CONFIGS["stress" if args.workload == "stress" else "perceive"]
     if os.environ.get("STP3_BENCH_DUMP_AFTER"):      # debugging aid: Python stacks of every thread after N seconds, then exit
         import faulthandler
@@ -462,6 +494,8 @@ def main():
         parallel.barrier()
         torch.cuda.synchronize()
 
+    last = {}
+
     def timed(fn, steps):
         evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         barrier()
@@ -479,7 +513,7 @@ def main():
             threading.Thread(target=watch, daemon=True).start()
         for s, e in evs:
             flush.zero_()                      # evict L2 between timed iterations (not timed)
-            s.record(); fn(); e.record()
+            s.record(); last["out"] = fn(); e.record()
             issued[0] += 1
         barrier()
         if stop is not None:
@@ -525,6 +559,8 @@ def main():
     if args.profiler_range:
         torch.cuda.synchronize()
         torch.cuda.cudart().cudaProfilerStop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last["out"], args.dump_outputs)
     e2e_mode = "serial: H2D -> compute -> D2H per step"
     if graphed is not None and not args.no_pipeline:
         from stp3_b200.models.stp3 import PipelinedPerception

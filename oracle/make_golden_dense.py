@@ -1,6 +1,8 @@
 """Generates tests/golden/dense_*.npz from the UNMODIFIED reference modules (TemporalModel, Decoder) run on CPU in the
-build container with deterministic weights (oracle.torch_dense.init_exact) and inputs.  Test infrastructure; run by
-hand:  python -m oracle.make_golden_dense"""
+build container with deterministic weights (oracle.torch_dense.init_exact) and inputs, and
+tests/golden/reference_state_dicts.json (the parameter names and shapes of those modules).  Test infrastructure; run
+by hand:  python -m oracle.make_golden_dense"""
+import json
 import os
 import sys
 
@@ -23,8 +25,26 @@ def dense_input(shape, seed):
     return TD.exact_gauss(shape, g)
 
 
+STATE_DICTS = "reference_state_dicts.json"
+
+
+def state_dict_shapes(module):
+    return {k: list(v.shape) for k, v in module.state_dict().items()}
+
+
+def write_state_dicts(ref):
+    """The checkpoint layout the drop-in modules must keep: TemporalModel(70, 3, (20, 20)) and the decoder with every
+    head on, Decoder(64, 2, 3, 2, GATES_ALL)."""
+    rec = {"temporal_model": state_dict_shapes(ref.temporal_model.TemporalModel(70, 3, (20, 20))),
+           "decoder_all": state_dict_shapes(ref.decoder.Decoder(64, 2, 3, 2, GATES_ALL))}
+    with open(os.path.join(OUT, STATE_DICTS), "w") as f:
+        json.dump(rec, f, indent=1)
+        f.write("\n")
+
+
 def main():
     ref = load_reference()
+    write_state_dicts(ref)
     torch.manual_seed(0)
     H, W = 24, 40
     with torch.no_grad():

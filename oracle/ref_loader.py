@@ -14,10 +14,10 @@ import types
 from types import SimpleNamespace
 
 _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-# the reference where it lies (build container), else its unmodified install under the git-ignored baseline/_ref/
-# (oracle/build_ref.py; that copy travels to the GPU box)
-_CANDIDATES = [os.environ.get("STP3_REFERENCE_ROOT"), "/root/reference", os.path.join(_REPO, "baseline", "_ref")]
-REFERENCE_ROOT = next((c for c in _CANDIDATES if c and os.path.isdir(os.path.join(c, "stp3"))), "/root/reference")
+# the reference checkout named by STP3_REFERENCE_ROOT, else its unmodified install under the git-ignored oracle/_ref/
+# (oracle/build_ref.py)
+_CANDIDATES = [os.environ.get("STP3_REFERENCE_ROOT"), os.path.join(_REPO, "oracle", "_ref")]
+REFERENCE_ROOT = next((c for c in _CANDIDATES if c and os.path.isdir(os.path.join(c, "stp3"))), _CANDIDATES[-1])
 
 
 def reference_available() -> bool:

@@ -1,6 +1,7 @@
 """CPU: pins oracle/torch_dense.py (the plain-PyTorch restatement used as the dense oracle on the GPU box) to
 (a) the golden outputs produced from the unmodified reference modules, using the drop-in modules purely as parameter
-containers, and (b) when /root/reference is present, the reference modules' own forward."""
+containers, and (b) the parameter names and shapes of the reference modules."""
+import json
 import os
 
 import numpy as np
@@ -8,7 +9,7 @@ import pytest
 import torch
 
 from oracle import torch_dense as TD
-from oracle.make_golden_dense import GATES_ALL, GATES_PERCEIVE, dense_input
+from oracle.make_golden_dense import GATES_ALL, GATES_PERCEIVE, STATE_DICTS, dense_input, state_dict_shapes
 from stp3_b200.models.decoder import Decoder
 from stp3_b200.models.temporal_model import TemporalModel
 from tests.helpers import GOLDEN
@@ -62,15 +63,10 @@ def test_decoder_restatement_matches_reference_output(name, gates):
 
 
 def test_state_dict_keys_match_reference_when_available():
-    from oracle.ref_loader import load_reference, reference_available
-    if not reference_available():
-        pytest.skip("/root/reference not present (GPU box)")
-    ref = load_reference()
-    a = TemporalModel(70, 3, (20, 20)).state_dict()
-    b = ref.temporal_model.TemporalModel(70, 3, (20, 20)).state_dict()
-    assert {k: v.shape for k, v in a.items()} == {k: v.shape for k, v in b.items()}
-    a = Decoder(64, 2, 3, 2, GATES_ALL).state_dict()
-    b = ref.decoder.Decoder(64, 2, 3, 2, GATES_ALL).state_dict()
-    assert {k: v.shape for k, v in a.items()} == {k: v.shape for k, v in b.items()}
-    # and the reference modules load the drop-in's checkpoint strictly
-    ref.decoder.Decoder(64, 2, 3, 2, GATES_ALL).load_state_dict(Decoder(64, 2, 3, 2, GATES_ALL).state_dict(), strict=True)
+    """The drop-in modules keep the reference's checkpoint layout: the same parameter and buffer names with the same
+    shapes as the reference modules had (tests/golden/reference_state_dicts.json, oracle/make_golden_dense.py), so a
+    reference checkpoint loads into them strictly and theirs into the reference."""
+    with open(os.path.join(GOLDEN, STATE_DICTS)) as f:
+        ref = json.load(f)
+    assert state_dict_shapes(TemporalModel(70, 3, (20, 20))) == ref["temporal_model"]
+    assert state_dict_shapes(Decoder(64, 2, 3, 2, GATES_ALL)) == ref["decoder_all"]
