@@ -144,7 +144,11 @@ typedef struct stp3_conv_desc {
   int res_cstride, res_coff;
   int n_valid;           /* real output channels written to y_f32 */
   int sigmoid;           /* apply a sigmoid to y_f32 (instance_center head, decoder.py:70) */
-  int tune_n_sub;        /* 0 = automatic; 1 / 2 = sub-tiles (8x16 pixels each) per CTA tile; 3 = 16x16 tile of a CTA pair (cta_group::2) */
+  int tune_n_sub;        /* 0 = automatic; 1 / 2 = sub-tiles (8x16 pixels each) per CTA tile; 3 = 16x16 tile of a CTA pair (cta_group::2);
+                            4 / 5 = linear tiling: 128 consecutive output pixels of the flattened (image, oy, ox) space per
+                            CTA / 256 per CTA pair, one im2col load per tap, bn = 256 in ONE launch.  Linear tiling takes
+                            2-D taps (dt = 0) over every frame (t0 = 0, T = T_total) and no col_sums, head, img_bias or
+                            y_f32 (STP3_EINVAL otherwise) */
   int tune_group;        /* 0 = automatic; 1 = never share an activation load between the dy taps of a 3x3; 3 = share;
                             +4 = stream the weights through the smem ring even if they would fit (more activation stages);
                             +8 = (bn 64) one stacked [W_hi; W_lo] operand: 2 MMAs per product instead of 3 */

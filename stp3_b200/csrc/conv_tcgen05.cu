@@ -99,21 +99,28 @@ struct ConvParams {
   // warp keeps running sums of its pixels in registers and writes one partial row per (CTA, lane quarter, image) --
   // plain stores, fixed order: deterministic.  BN = 64 only.  sum_part: [gridDim.x][4][n_img][BN], zeroed by the host.
   float* sum_part;
+  // linear tiling (LINEAR = true): a tile is 128 (256 for a pair) consecutive output pixels of the flattened
+  // (image, oy, ox) space; one im2col TMA load per (tap, K block) brings them, zero-filled outside the image
+  int m_total;              // n_img * Ho * Wo
+  int lin_lo_w, lin_lo_h;   // lower corner of the im2col bounding box (smallest tap offset); a tap loads at d - lo
+  // work units: (tile, column half); n_halves = 2 runs a 256-column convolution in one launch (linear tiling only)
+  int n_halves, n_units;
 };
 
 // STACK (BN = 64 only): the hi and lo weight planes of a K step form ONE B operand of 2*BN rows, so a product is two
 // MMAs instead of three -- A_hi x [W_hi; W_lo] (N = 2*BN) and A_lo x W_hi (N = BN) -- and the activation tile is read
 // from shared memory twice instead of three times (N = 64 MMAs are bound by exactly those reads).  The accumulator
 // has 2*BN columns; the epilogue adds columns c and BN + c.
-template <int BN, bool PAIR = false, bool STACK = false>
+template <int BN, bool PAIR = false, bool STACK = false, bool LINEAR = false>
 struct ConvSmem {
   static constexpr int kBRows = PAIR ? BN / 2 : BN;                    // weight rows held by one CTA (a pair splits N)
   // B_hi + B_lo of one K step; a stacked pair holds [own half of the stacked operand (BN rows)][own half of W_hi]
   static constexpr int kBTileBytes = (STACK && PAIR ? 3 : 2) * kBRows * kBK * 2;
   static constexpr int kAccCols = STACK ? 2 * BN : BN;                 // TMEM columns of one accumulator
   static constexpr int kTmemCols = 4 * kAccCols;                       // 2 sub-tiles x 2 accumulator buffers
+  static constexpr int kBiasCols = LINEAR ? 2 * BN : BN;               // bias of both column halves
   static constexpr size_t tail_bytes() {
-    return (1 + kMaxHeadOut) * BN * sizeof(float) + kMaxHeadOut * 128 * sizeof(float) + kEpiWarps * 64 * sizeof(float) +
+    return (kBiasCols + kMaxHeadOut * BN) * sizeof(float) + kMaxHeadOut * 128 * sizeof(float) + kEpiWarps * 64 * sizeof(float) +
            (2 * kMaxAStages + 2 * kMaxBStages + 8) * 8;
   }
 };
@@ -145,11 +152,19 @@ __device__ __forceinline__ bool group_is_padding(const ConvParams& p, int grp, i
 // operand reads per MMA drop by a quarter and the weight traffic per SM halves.  Barrier protocol: "full" barriers
 // live in the leader and collect the TMA bytes of both CTAs; "empty" / "accumulator ready" are multicast commits;
 // "accumulator drained" collects the epilogue warps of both CTAs in the leader.
-template <int BN, bool PAIR, bool STACK>
+//
+// LINEAR = true: a tile is 128 consecutive output pixels of the flattened (image, oy, ox) space per CTA (256 for a
+// pair; n_sub = 1), so rows and images are crossed and only the tail of the last tile is wasted -- small maps (50^2,
+// 25^2) otherwise compute up to 39 % padding pixels in 16x16 tiles.  tm_a_hi / tm_a_lo are rank-4 im2col maps; every
+// (tap, K block) is its own A load (no dy sharing), issued in the same (group, K block, tap) order as the 2-D tiling
+// so each pixel accumulates the same products in the same order.  A work unit is (tile, column half): a 256-column
+// convolution walks both halves in one launch.
+template <int BN, bool PAIR, bool STACK, bool LINEAR>
 __global__ void __launch_bounds__(kConvThreads, 1)
 conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
                   const __grid_constant__ CUtensorMap tm_w, const ConvParams p) {
-  using S = ConvSmem<BN, PAIR, STACK>;
+  using S = ConvSmem<BN, PAIR, STACK, LINEAR>;
+  constexpr int kLinTile = PAIR ? 256 : 128;      // output pixels of a linear tile
   static_assert(!STACK || BN == 64, "stacked weight operand: BN = 64 only (TMEM columns)");
   const int kBRows = p.b_rows;
   const uint32_t rank = PAIR ? ptx::cluster_ctarank() : 0u;              // 0 = leader
@@ -165,7 +180,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
   unsigned char* a_ring = smem;
   unsigned char* b_ring = a_ring + (size_t)p.na_stages * a_stage_bytes;            // ring, or the resident weights
   float* s_bias = reinterpret_cast<float*>(b_ring + (size_t)(resident ? k_iters : p.nb_stages) * p.b_tile_bytes);
-  float* s_head = s_bias + BN;                    // [kMaxHeadOut][BN]
+  float* s_head = s_bias + S::kBiasCols;          // [kMaxHeadOut][BN]
   float* s_hx = s_head + kMaxHeadOut * BN;        // [kMaxHeadOut][128] head partials handed between column halves
   float* s_wb = s_hx + kMaxHeadOut * 128;         // [kEpiWarps][64] per-image bias slice of each epilogue warp
   uint64_t* bars = reinterpret_cast<uint64_t*>(s_wb + kEpiWarps * 64);
@@ -199,7 +214,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
     if constexpr (PAIR) ptx::tmem_alloc_pair<S::kTmemCols>(tmem_slot);
     else ptx::tmem_alloc<S::kTmemCols>(tmem_slot);
   }
-  for (int i = threadIdx.x; i < BN; i += blockDim.x) s_bias[i] = p.bias[i];
+  for (int i = threadIdx.x; i < BN * p.n_halves; i += blockDim.x) s_bias[i] = p.bias[i];
   for (int i = threadIdx.x; i < p.head_ko * BN; i += blockDim.x) s_head[i] = p.head_w[i];
   ptx::tc_fence_before();
   __syncthreads();
@@ -209,14 +224,16 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
   const int tiles_per_img = p.tiles_x * p.tiles_y;
   const int n_groups = p.n_groups;
   const int tile_h = PAIR ? 2 * kSubH : kSubH * p.n_sub;      // image rows of a tile (a pair: 8 per CTA)
+  const int hw_out = p.Ho * p.Wo;
 
   if (warp == 0) {
     // ===================== TMA producer (whole warp walks the loops; one elected lane issues) =====================
     {
       // in a pair every "full" barrier is the leader's: arrive / complete_tx go through its shared::cluster address.
       // load_b: the weight tile of K step `it` into `dst` (called by the elected lane; transaction bytes on `bar`)
+      int w_row_off = p.w_row_off;                // + BN for the upper column half of a work unit
       auto load_b = [&](unsigned char* dst, int it, uint64_t* bar) {
-        const int row_hi = (it * 2) * p.w_rows + p.w_row_off, row_lo = row_hi + p.w_rows;
+        const int row_hi = (it * 2) * p.w_rows + w_row_off, row_lo = row_hi + p.w_rows;
         if constexpr (PAIR) {
           const uint32_t cbar = ptx::mapa(ptx::smem_u32(bar), 0);
           if constexpr (STACK) {
@@ -245,22 +262,49 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
       __syncwarp();
       ptx::griddep_wait();                        // activations come from the preceding kernel
       int as = 0, bs = 0; uint32_t aph = 0, bph = 0;
-      for (int tile = cta; tile < p.n_tiles; tile += n_cta) {
-        const int img = tile / tiles_per_img, rem = tile % tiles_per_img;
-        const int oy0 = (rem / p.tiles_x) * tile_h + (int)rank * kSubH, ox0 = (rem % p.tiles_x) * kTileW;
+      for (int unit = cta; unit < p.n_units; unit += n_cta) {
+        const int tile = LINEAR ? unit / p.n_halves : unit;
+        if constexpr (LINEAR) w_row_off = p.w_row_off + (unit % p.n_halves) * BN;
+        int img, oy0, ox0;                        // first output pixel this CTA loads
+        if constexpr (LINEAR) {
+          int m = tile * kLinTile + (int)rank * 128;
+          if (m >= p.m_total) m = 0;              // the peer's rows of a last pair tile: loaded, never stored
+          img = m / hw_out;
+          const int rem = m - img * hw_out;
+          oy0 = rem / p.Wo; ox0 = rem - oy0 * p.Wo;
+        } else {
+          img = tile / tiles_per_img;
+          const int rem = tile % tiles_per_img;
+          oy0 = (rem / p.tiles_x) * tile_h + (int)rank * kSubH; ox0 = (rem % p.tiles_x) * kTileW;
+        }
         const int bidx = img / p.T, tidx = p.t0 + img % p.T;
         for (int grp = 0; grp < n_groups; ++grp) {
           const int tap0 = p.gstart[grp], gsz = p.gsize[grp];
-          const int x = ox0 * p.stride + p.tap[tap0][2];
-          const int y = oy0 * p.stride + p.tap[tap0][1];
+          // linear: the start of the traversal inside the im2col bounding box; the tap travels as the load's offset
+          const int x = ox0 * p.stride + (LINEAR ? p.lin_lo_w : p.tap[tap0][2]);
+          const int y = oy0 * p.stride + (LINEAR ? p.lin_lo_h : p.tap[tap0][1]);
           const int t = tidx + p.tap[tap0][0];
-          if (p.skip_t && group_is_padding(p, grp, tidx, oy0 - (int)rank * kSubH, ox0, tile_h)) continue;
-          for (int kb = 0; kb < p.kblocks; ++kb) {
+          if (!LINEAR && p.skip_t && group_is_padding(p, grp, tidx, oy0 - (int)rank * kSubH, ox0, tile_h)) continue;
+          // the activation stage of tap group member j (linear: its own im2col load; 2-D: one box for the group)
+          auto load_a = [&](int kb, int j) {
             ptx::mbar_wait(&a_empty[as], aph ^ 1);
             if (ptx::elect_one_sync()) {
               unsigned char* sa = a_ring + (size_t)as * a_stage_bytes;
               const int c = p.cin_off + kb * kBK;
-              if constexpr (PAIR) {
+              if constexpr (LINEAR) {
+                const uint16_t ow = (uint16_t)(p.tap[tap0 + j][2] - p.lin_lo_w);
+                const uint16_t oh = (uint16_t)(p.tap[tap0 + j][1] - p.lin_lo_h);
+                if constexpr (PAIR) {
+                  const uint32_t bar = ptx::mapa(ptx::smem_u32(&a_full[as]), 0);
+                  ptx::mbar_arrive_expect_tx_cluster(bar, (uint32_t)a_stage_bytes);
+                  ptx::tma_load_im2col_4d_pair(sa, &tm_a_hi, bar, c, x, y, img, ow, oh);
+                  ptx::tma_load_im2col_4d_pair(sa + p.a_plane_bytes, &tm_a_lo, bar, c, x, y, img, ow, oh);
+                } else {
+                  ptx::mbar_arrive_expect_tx(&a_full[as], (uint32_t)a_stage_bytes);
+                  ptx::tma_load_im2col_4d(sa, &tm_a_hi, &a_full[as], c, x, y, img, ow, oh);
+                  ptx::tma_load_im2col_4d(sa + p.a_plane_bytes, &tm_a_lo, &a_full[as], c, x, y, img, ow, oh);
+                }
+              } else if constexpr (PAIR) {
                 const uint32_t bar = ptx::mapa(ptx::smem_u32(&a_full[as]), 0);
                 ptx::mbar_arrive_expect_tx_cluster(bar, (uint32_t)a_stage_bytes);
                 ptx::tma_load_5d_pair(sa, &tm_a_hi, bar, c, x, y, t, bidx);
@@ -273,17 +317,26 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
             }
             __syncwarp();
             if (++as == p.na_stages) { as = 0; aph ^= 1; }
-            if (!resident) {
-              for (int j = 0; j < gsz; ++j) {
-                const int it = (tap0 + j) * p.kblocks + kb;          // [tap][kb][plane][rows] blocks of 64-wide rows
-                ptx::mbar_wait(&b_empty[bs], bph ^ 1);
-                if (ptx::elect_one_sync()) {
-                  expect_b(&b_full[bs], (uint32_t)p.b_tile_bytes);
-                  load_b(b_ring + (size_t)bs * p.b_tile_bytes, it, &b_full[bs]);
-                }
-                __syncwarp();
-                if (++bs == p.nb_stages) { bs = 0; bph ^= 1; }
+          };
+          auto load_w = [&](int kb, int j) {
+            const int it = (tap0 + j) * p.kblocks + kb;              // [tap][kb][plane][rows] blocks of 64-wide rows
+            ptx::mbar_wait(&b_empty[bs], bph ^ 1);
+            if (ptx::elect_one_sync()) {
+              expect_b(&b_full[bs], (uint32_t)p.b_tile_bytes);
+              load_b(b_ring + (size_t)bs * p.b_tile_bytes, it, &b_full[bs]);
+            }
+            __syncwarp();
+            if (++bs == p.nb_stages) { bs = 0; bph ^= 1; }
+          };
+          for (int kb = 0; kb < p.kblocks; ++kb) {
+            if constexpr (LINEAR) {
+              for (int j = 0; j < gsz; ++j) {                        // A and W of each tap in turn: the issuer
+                load_a(kb, j);                                       // consumes them in this order
+                if (!resident) load_w(kb, j);
               }
+            } else {
+              load_a(kb, 0);
+              if (!resident) for (int j = 0; j < gsz; ++j) load_w(kb, j);
             }
           }
         }
@@ -307,22 +360,31 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
       if (resident) wait_full(bres_bar, 0);
       int as = 0, bs = 0; uint32_t aph = 0, bph = 0;
       int buf = 0; uint32_t acc_phase = 0;
-      for (int tile = cta; tile < p.n_tiles; tile += n_cta) {
+      for (int unit = cta; unit < p.n_units; unit += n_cta) {
         wait_full(&tmem_empty_bar[buf], acc_phase ^ 1);           // the epilogue has drained this accumulator pair
         ptx::tc_fence_after();
         uint32_t accumulate = 0;
+        const int tile = LINEAR ? unit / p.n_halves : unit;
         const int tidx = p.t0 + (tile / tiles_per_img) % p.T;
         const int rem_m = tile % tiles_per_img;
         const int oy_m = (rem_m / p.tiles_x) * tile_h, ox_m = (rem_m % p.tiles_x) * kTileW;
         for (int grp = 0; grp < n_groups; ++grp) {
-          if (p.skip_t && group_is_padding(p, grp, tidx, oy_m, ox_m, tile_h)) continue;
+          if (!LINEAR && p.skip_t && group_is_padding(p, grp, tidx, oy_m, ox_m, tile_h)) continue;
           const int tap0 = p.gstart[grp], gsz = p.gsize[grp];
           for (int kb = 0; kb < p.kblocks; ++kb) {
-            wait_full(&a_full[as], aph);
-            ptx::tc_fence_after();
             const int k_begin = kb == 0 ? p.ks_first : 0, k_end = kb == p.kblocks - 1 ? p.ks_end : kBK / 16;
-            const uint32_t a_hi0 = ptx::smem_u32(a_ring + (size_t)as * a_stage_bytes);
+            uint32_t a_hi0 = 0;
+            if constexpr (!LINEAR) {                     // one activation stage serves the whole group
+              wait_full(&a_full[as], aph);
+              ptx::tc_fence_after();
+              a_hi0 = ptx::smem_u32(a_ring + (size_t)as * a_stage_bytes);
+            }
             for (int j = 0; j < gsz; ++j) {
+              if constexpr (LINEAR) {                    // one activation stage per tap
+                wait_full(&a_full[as], aph);
+                ptx::tc_fence_after();
+                a_hi0 = ptx::smem_u32(a_ring + (size_t)as * a_stage_bytes);
+              }
               const int it = (tap0 + j) * p.kblocks + kb;
               uint32_t b_hi;
               if (resident) {
@@ -338,7 +400,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
               if (ptx::elect_one_sync()) {
               for (int sub = 0; sub < (PAIR ? 1 : p.n_sub); ++sub) {
                 // sub-tile rows [sub*8, sub*8+8) of the tile, shifted by j image rows inside the loaded box
-                const uint32_t a_hi = a_hi0 + (uint32_t)((j * kTileW + sub * 128) * 128);
+                const uint32_t a_hi = a_hi0 + (uint32_t)(((LINEAR ? 0 : j * kTileW) + sub * 128) * 128);
                 const uint64_t da_hi = ptx::umma_desc_k_sw128(a_hi), da_lo = ptx::umma_desc_k_sw128(a_hi + p.a_plane_bytes);
                 const uint32_t tmem_d = tmem_base + (uint32_t)((buf * 2 + sub) * S::kAccCols);
 #pragma unroll
@@ -361,10 +423,17 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
               __syncwarp();
               accumulate = 1;
               if (!resident) { if (++bs == p.nb_stages) { bs = 0; bph ^= 1; } }
+              if constexpr (LINEAR) {
+                if (ptx::elect_one_sync()) commit(&a_empty[as]);                // frees the activation slot
+                __syncwarp();
+                if (++as == p.na_stages) { as = 0; aph ^= 1; }
+              }
             }
-            if (ptx::elect_one_sync()) commit(&a_empty[as]);                    // frees the activation slot
-            __syncwarp();
-            if (++as == p.na_stages) { as = 0; aph ^= 1; }
+            if constexpr (!LINEAR) {
+              if (ptx::elect_one_sync()) commit(&a_empty[as]);                  // frees the activation slot
+              __syncwarp();
+              if (++as == p.na_stages) { as = 0; aph ^= 1; }
+            }
           }
         }
         if (ptx::elect_one_sync()) commit(&tmem_full_bar[buf]);                 // accumulators complete -> epilogue
@@ -415,9 +484,25 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
       }
     };
     ptx::griddep_wait();                          // residual / per-image bias reads and every global write come after
-    for (int tile = cta; tile < p.n_tiles; tile += n_cta) {
-      const int img = tile / tiles_per_img, rem = tile % tiles_per_img;
-      const int oy_t = (rem / p.tiles_x) * tile_h + (int)rank * kSubH, ox = (rem % p.tiles_x) * kTileW + (r & 15);
+    for (int unit = cta; unit < p.n_units; unit += n_cta) {
+      const int tile = LINEAR ? unit / p.n_halves : unit;
+      const int ucoff = LINEAR ? (unit % p.n_halves) * BN : 0;   // first column of this unit's half of the convolution
+      const int u_coff = d_coff + ucoff, u_nstore = d_nstore - ucoff;
+      // 2-D: image of the tile, first image row of this CTA's part and this lane's column; linear: this lane's pixel
+      // (img >= n_img past the last pixel)
+      int img, oy_t, ox;
+      if constexpr (LINEAR) {
+        const int m = tile * kLinTile + (int)rank * 128 + r;
+        img = m / hw_out;
+        const int rem = m - img * hw_out;
+        oy_t = rem / p.Wo; ox = rem - oy_t * p.Wo;
+      } else {
+        img = tile / tiles_per_img;
+        const int rem = tile % tiles_per_img;
+        oy_t = (rem / p.tiles_x) * tile_h + (int)rank * kSubH; ox = (rem % p.tiles_x) * kTileW + (r & 15);
+      }
+      auto row_of = [&](int sub) { return LINEAR ? oy_t : oy_t + sub * kSubH + (r >> 4); };
+      auto stored = [&](int oy) { return LINEAR ? img < p.n_img : oy < p.Ho && ox < p.Wo; };
       if (kSums && p.sum_part && img != sum_img) {      // tiles come in image order: hand the finished image over
         if (sum_img >= 0) flush_sums(sum_img);
         sum_img = img;
@@ -427,9 +512,9 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
       const int n_sub_eff = PAIR ? 1 : p.n_sub;
       uint32_t nh[8], nl[8];
       auto request_residual = [&](int sub, int j) {
-        const int oy = oy_t + sub * kSubH + (r >> 4);
-        if (oy < p.Ho && ox < p.Wo) {
-          const size_t off = (((size_t)img * p.Ho + oy) * p.Wo + ox) * p.res_cstride + p.res_coff + col0 + j * 16;
+        const int oy = row_of(sub);
+        if (stored(oy)) {
+          const size_t off = (((size_t)img * p.Ho + oy) * p.Wo + ox) * p.res_cstride + p.res_coff + ucoff + col0 + j * 16;
           // coherent loads: the residual (like the per-image bias below) is written by a PRECEDING kernel that this grid
           // may overlap under programmatic dependent launch, so the read-only (.nc) path is not allowed for it
           if (p.vec256 & 2) {
@@ -447,7 +532,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
         }
       };
       if (p.res_mode) request_residual(0, 0);
-      const float* bsrc = s_bias;                 // bias of column c at bsrc[c]
+      const float* bsrc = s_bias + ucoff;         // bias of column c at bsrc[c]
       if (p.img_bias) {
         const float* ib = p.img_bias + (size_t)img * p.img_bias_stride + col0;
         float* wb = s_wb + e * 64;
@@ -461,8 +546,8 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
       ptx::tc_fence_after();
 #pragma unroll 1
       for (int sub = 0; sub < n_sub_eff; ++sub) {
-        const int oy = oy_t + sub * kSubH + (r >> 4);
-        const bool valid = oy < p.Ho && ox < p.Wo;
+        const int oy = row_of(sub);
+        const bool valid = stored(oy);
         const size_t pix = ((size_t)img * p.Ho + oy) * p.Wo + ox;
         float hacc[kMaxHeadOut];
 #pragma unroll
@@ -520,9 +605,9 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
 #pragma unroll
               for (int i = 0; i < 16; ++i) v[i] = fmaxf(v[i], 0.f);
             }
-            if (d_hi && cb < d_nstore) {
-              __nv_bfloat16* ohp = d_hi + pix * d_cstride + d_coff + cb;
-              __nv_bfloat16* olp = d_lo + pix * d_cstride + d_coff + cb;
+            if (d_hi && cb < u_nstore) {
+              __nv_bfloat16* ohp = d_hi + pix * d_cstride + u_coff + cb;
+              __nv_bfloat16* olp = d_lo + pix * d_cstride + u_coff + cb;
               uint32_t hw[8], lw[8];
 #pragma unroll
               for (int e2 = 0; e2 < 8; ++e2) {
@@ -532,20 +617,20 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
                 hw[e2] = h;
                 lw[e2] = ptx::pack_bf16x2(r0, r1);
               }
-              if (d_vec && cb + 16 <= d_nstore) {               // one full 32-byte sector per plane and lane
+              if (d_vec && cb + 16 <= u_nstore) {               // one full 32-byte sector per plane and lane
                 ptx::st_global_v8(ohp, hw);
                 ptx::st_global_v8(olp, lw);
               } else {
                 reinterpret_cast<uint4*>(ohp)[0] = make_uint4(hw[0], hw[1], hw[2], hw[3]);
                 reinterpret_cast<uint4*>(olp)[0] = make_uint4(lw[0], lw[1], lw[2], lw[3]);
-                if (cb + 8 < d_nstore) {
+                if (cb + 8 < u_nstore) {
                   reinterpret_cast<uint4*>(ohp)[1] = make_uint4(hw[4], hw[5], hw[6], hw[7]);
                   reinterpret_cast<uint4*>(olp)[1] = make_uint4(lw[4], lw[5], lw[6], lw[7]);
                 }
               }
             }
             if (p.out_f32 && p.f32_nhwc) {
-              const int c0 = p.f32_coff + cb;
+              const int c0 = p.f32_coff + ucoff + cb;
               float* dst = p.out_f32 + pix * p.n_valid + c0;
               if (c0 + 16 <= p.n_valid && (p.n_valid & 7) == 0) {          // rows are 32-byte aligned (host checks the base)
                 ptx::st_global_v8f(dst, v);
@@ -558,7 +643,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_cons
             } else if (p.out_f32) {
 #pragma unroll
               for (int i = 0; i < 16; ++i) {
-                const int c = p.f32_coff + cb + i;
+                const int c = p.f32_coff + ucoff + cb + i;
                 if (c < p.n_valid) {
                   float x = v[i];
                   if (p.sigmoid) x = 1.f / (1.f + __expf(-x));
@@ -677,6 +762,23 @@ static PFN_tmapEncodeTiled encode_fn() {
   return fn;
 }
 
+typedef CUresult (*PFN_tmapEncodeIm2col)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                         const cuuint64_t*, const int*, const int*, cuuint32_t, cuuint32_t,
+                                         const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                         CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+static PFN_tmapEncodeIm2col encode_im2col_fn() {
+  static PFN_tmapEncodeIm2col fn = nullptr;
+  if (!fn) {
+    void* ptr = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeIm2col", &ptr, cudaEnableDefault, &qres) == cudaSuccess &&
+        qres == cudaDriverEntryPointSuccess)
+      fn = reinterpret_cast<PFN_tmapEncodeIm2col>(ptr);
+  }
+  return fn;
+}
+
 int launch_col_sum_reduce(const float* part, int n_part, int n_img, float* out, cudaStream_t stream) {
   STP3_CUDA_OK(launch_pdl(col_sum_reduce_kernel, dim3(n_img), dim3(64, 16), 0, stream, part, n_part, n_img, 64, out));
   return STP3_OK;
@@ -760,13 +862,50 @@ extern "C" int stp3_conv_fwd(const stp3_conv_desc* d, const void* x_hi, const vo
   const long long tiles16 = (long long)n_img_ * ceil_div(d->Wo, kTileW) * ceil_div(d->Ho, 2 * kSubH);
   // tune_n_sub == 3: the 16x16 tile is shared by a CTA pair (cta_group::2), 8 image rows per CTA
   // untuned (tune_n_sub == 0) multi-tap layers take the pair tiling, the autotuner's choice on all of them
-  const bool pair = want_nsub == 3 || (want_nsub == 0 && d->ntaps > 1);
-  const int n_sub = pair ? 1 : (want_nsub == 1 || want_nsub == 2 ? want_nsub : (tiles16 >= 3 * 148 ? 2 : 1));
+  // tune_n_sub == 4 / 5: linear tiling, 128 consecutive output pixels per CTA / 256 per CTA pair (see the kernel)
+  const bool linear = want_nsub == 4 || want_nsub == 5;
+  const bool pair = want_nsub == 3 || want_nsub == 5 || (want_nsub == 0 && d->ntaps > 1);
+  const int n_sub = pair || linear ? 1 : (want_nsub == 1 || want_nsub == 2 ? want_nsub : (tiles16 >= 3 * 148 ? 2 : 1));
   const int tile_h = pair ? 2 * kSubH : kSubH * n_sub;
   const int box_h = kSubH * n_sub + (group - 1);                         // image rows one CTA loads per stage
 
   CUtensorMap tm_hi, tm_lo, tm_w;
-  {
+  int lin_lo_w = 0, lin_lo_h = 0;
+  if (linear) {
+    STP3_CHECK_ARG(d->t0 == 0 && d->T == T_total, "linear tiling: every frame of the input tensor (no frame window)");
+    STP3_CHECK_ARG(!d->col_sums && !head && !img_bias && !y_f32,
+                   "linear tiling: no col_sums, fused head, per-image bias or fp32 output");
+    int hi_w = d->taps[0][2], hi_h = d->taps[0][1];
+    lin_lo_w = hi_w; lin_lo_h = hi_h;
+    for (int i = 0; i < d->ntaps; ++i) {
+      STP3_CHECK_ARG(d->taps[i][0] == 0, "linear tiling: 2-D taps only (dt = 0)");
+      lin_lo_w = d->taps[i][2] < lin_lo_w ? d->taps[i][2] : lin_lo_w; hi_w = d->taps[i][2] > hi_w ? d->taps[i][2] : hi_w;
+      lin_lo_h = d->taps[i][1] < lin_lo_h ? d->taps[i][1] : lin_lo_h; hi_h = d->taps[i][1] > hi_h ? d->taps[i][1] : hi_h;
+    }
+    // bounding box of the traversal: the first input pixel of every output pixel's window (tap at the lower corner),
+    // [lo, dim - 1 + up] walked with the conv stride, so that it holds exactly Wo x Ho start pixels
+    const int up_w = (d->Wo - 1) * d->stride + lin_lo_w - (d->W - 1);
+    const int up_h = (d->Ho - 1) * d->stride + lin_lo_h - (d->H - 1);
+    auto in8 = [](int v) { return v >= -128 && v <= 127; };
+    STP3_CHECK_ARG(in8(lin_lo_w) && in8(lin_lo_h) && in8(up_w) && in8(up_h) && hi_w - lin_lo_w < 256 &&
+                   hi_h - lin_lo_h < 256, "linear tiling: padding / output size outside the im2col corner range [-128, 127]");
+    PFN_tmapEncodeIm2col enc2 = encode_im2col_fn();
+    if (!enc2) return set_error(STP3_ECUDA, "cuTensorMapEncodeIm2col is not available from the driver");
+    const cuuint64_t dims[4] = {(cuuint64_t)d->in_cstride, (cuuint64_t)d->W, (cuuint64_t)d->H,
+                                (cuuint64_t)d->B * T_total};
+    const cuuint64_t strides[3] = {(cuuint64_t)d->in_cstride * 2, (cuuint64_t)d->W * d->in_cstride * 2,
+                                   (cuuint64_t)d->H * d->W * d->in_cstride * 2};
+    const int lower[2] = {lin_lo_w, lin_lo_h}, upper[2] = {up_w, up_h};          // innermost (W) first
+    const cuuint32_t estr[4] = {1, (cuuint32_t)d->stride, (cuuint32_t)d->stride, 1};
+    CUresult r1 = enc2(&tm_hi, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x_hi), dims, strides, lower, upper,
+                       kBK, 128, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                       CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    CUresult r2 = enc2(&tm_lo, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x_lo), dims, strides, lower, upper,
+                       kBK, 128, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                       CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r1 != CUDA_SUCCESS || r2 != CUDA_SUCCESS)
+      return set_error(STP3_ECUDA, "cuTensorMapEncodeIm2col(activation) failed: %d %d", (int)r1, (int)r2);
+  } else {
     const cuuint64_t dims[5] = {(cuuint64_t)d->in_cstride, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)T_total,
                                 (cuuint64_t)d->B};
     const cuuint64_t strides[4] = {(cuuint64_t)d->in_cstride * 2, (cuuint64_t)d->W * d->in_cstride * 2,
@@ -785,7 +924,8 @@ extern "C" int stp3_conv_fwd(const stp3_conv_desc* d, const void* x_hi, const vo
       return set_error(STP3_ECUDA, "cuTensorMapEncodeTiled(activation) failed: %d %d", (int)r1, (int)r2);
   }
   const int kblocks = d->cin / kBK;
-  const int bn_launch = d->bn == 256 ? 128 : d->bn;     // 256 output channels run as two 128-column launches
+  const int bn_launch = d->bn == 256 ? 128 : d->bn;     // 256 output channels: two 128-column launches (2-D tiling)
+  const int n_halves = linear && d->bn == 256 ? 2 : 1;  // or one linear launch whose work units cover both halves
   // the MMAs cover only the columns that carry weights (n_cols, rounded up to the UMMA granularity of 16)
   const int n_mma = d->bn <= 128 && d->n_cols > 0 && d->n_cols < d->bn ? ((d->n_cols + 15) / 16) * 16 : bn_launch;
   {
@@ -804,6 +944,7 @@ extern "C" int stp3_conv_fwd(const stp3_conv_desc* d, const void* x_hi, const vo
   p.H = d->H; p.W = d->W;
   p.skip_t = 0;                                     // safe only if some tap always stays inside: the centre tap
   for (int i = 0; i < d->ntaps; ++i) if (d->taps[i][0] == 0 && d->taps[i][1] == 0 && d->taps[i][2] == 0) p.skip_t = 1;
+  p.m_total = 0; p.lin_lo_w = lin_lo_w; p.lin_lo_h = lin_lo_h; p.n_halves = n_halves;
   p.tiles_x = ceil_div(d->Wo, kTileW); p.tiles_y = ceil_div(d->Ho, tile_h); p.n_sub = n_sub;
   p.stride = d->stride; p.kblocks = kblocks; p.cin_off = d->cin_off; p.ntaps = d->ntaps;
   {
@@ -814,7 +955,7 @@ extern "C" int stp3_conv_fwd(const stp3_conv_desc* d, const void* x_hi, const vo
     p.ks_end = (k_hi - (kblocks - 1) * kBK) / 16;
     STP3_CHECK_ARG(kblocks > 1 || p.ks_first < p.ks_end, "empty K range");
   }
-  p.a_plane_bytes = box_h * kTileW * kBK * 2; p.w_rows = d->bn; p.n_mma = n_mma;
+  p.a_plane_bytes = (linear ? 128 : box_h * kTileW) * kBK * 2; p.w_rows = d->bn; p.n_mma = n_mma;
   for (int i = 0; i < d->ntaps; ++i) { p.tap[i][0] = d->taps[i][0]; p.tap[i][1] = d->taps[i][1]; p.tap[i][2] = d->taps[i][2]; p.tap[i][3] = 0; }
   p.relu = d->relu; p.res_mode = d->res_mode;
   p.res_hi = static_cast<const __nv_bfloat16*>(res_hi); p.res_lo = static_cast<const __nv_bfloat16*>(res_lo);
@@ -845,9 +986,11 @@ extern "C" int stp3_conv_fwd(const stp3_conv_desc* d, const void* x_hi, const vo
     for (int k = 0; k < head->n_out; ++k) { p.head_out[k] = head->out[k]; p.head_img_stride[k] = head->img_stride[k]; }
   }
   const int k_iters = d->ntaps * kblocks;
-  const long long nblk = (long long)p.n_img * p.tiles_x * p.tiles_y;
-  STP3_CHECK_ARG(nblk > 0 && nblk < (1ll << 31), "grid too large");
-  p.n_tiles = (int)nblk;
+  const long long m_total = (long long)p.n_img * d->Ho * d->Wo;
+  const long long n_tiles = linear ? (m_total + (pair ? 255 : 127)) / (pair ? 256 : 128) : (long long)p.n_img * p.tiles_x * p.tiles_y;
+  const long long nblk = n_tiles * n_halves;                                    // work units
+  STP3_CHECK_ARG(nblk > 0 && m_total < (1ll << 31) && nblk < (1ll << 31), "grid too large");
+  p.n_tiles = (int)n_tiles; p.n_units = (int)nblk; p.m_total = (int)m_total;
   const int num_sms = conv_num_sms();
   unsigned grid = (unsigned)(nblk < num_sms ? nblk : num_sms);           // persistent: one CTA per SM
   if (pair) grid = 2u * (unsigned)(nblk < num_sms / 2 ? nblk : num_sms / 2);
@@ -865,28 +1008,28 @@ extern "C" int stp3_conv_fwd(const stp3_conv_desc* d, const void* x_hi, const vo
     STP3_CUDA_OK(cudaMemsetAsync(p.sum_part, 0, (size_t)grid * 4 * p.n_img * 64 * sizeof(float), stream));
   }
 
-  for (int part = 0; part * bn_launch < d->bn; ++part) {
+  for (int part = 0; part * bn_launch * n_halves < d->bn; ++part) {
     const int coff = part * bn_launch;
     p.w_row_off = coff;
     p.bias = bias + coff;
     p.img_bias = img_bias ? img_bias + coff : nullptr;
     p.res_coff = d->res_coff + coff;
     p.out_coff = d->out_coff + coff;
-    p.n_store = n_store - coff < bn_launch ? (n_store - coff > 0 ? n_store - coff : 0) : bn_launch;
+    p.n_store = n_store - coff < bn_launch * n_halves ? (n_store - coff > 0 ? n_store - coff : 0) : bn_launch * n_halves;
     p.f32_coff = coff;
     auto al32 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 31) == 0; };
     p.vec256 = (y_hi && d->out_cstride % 16 == 0 && p.out_coff % 16 == 0 && al32(y_hi) && al32(y_lo) ? 1 : 0) |
                (d->res_mode && d->res_cstride % 16 == 0 && p.res_coff % 16 == 0 && al32(res_hi) && al32(res_lo) ? 2 : 0) |
                (d->y2_hi && d->out2_cstride % 16 == 0 && d->out2_coff % 16 == 0 && al32(d->y2_hi) && al32(d->y2_lo) ? 4 : 0);
-#define STP3_LAUNCH_CONV(BN_, PAIR_, STACK_)                                                                      \
+#define STP3_LAUNCH_CONV(BN_, PAIR_, STACK_, LIN_)                                                                \
     do {                                                                                                          \
-      using SM = ConvSmem<BN_, PAIR_, STACK_>;                                                                    \
+      using SM = ConvSmem<BN_, PAIR_, STACK_, LIN_>;                                                                  \
       p.b_rows = PAIR_ ? n_mma / 2 : n_mma;                                                                       \
       p.b_tile_bytes = (STACK_ && PAIR_ ? 3 : 2) * p.b_rows * kBK * 2;                                            \
       const size_t avail = smem_cap - 1024 - SM::tail_bytes();                                                    \
       const size_t wbytes = (size_t)k_iters * (size_t)p.b_tile_bytes;                                                    \
       /* small weight tensors stay resident in smem next to >= 2 activation stages */                            \
-      const bool res = !stream_weights && wbytes + 2 * a_stage <= avail;                                          \
+      const bool res = !stream_weights && n_halves == 1 && wbytes + 2 * a_stage <= avail;                                        \
       int na, nb;                                                                                                 \
       if (res) {                                                                                                  \
         na = (int)((avail - wbytes) / a_stage); nb = 0;                                                           \
@@ -904,7 +1047,7 @@ extern "C" int stp3_conv_fwd(const stp3_conv_desc* d, const void* x_hi, const vo
       if (nb > kMaxBStages) nb = kMaxBStages;                                                                     \
       p.na_stages = na; p.nb_stages = nb; p.b_resident = res ? 1 : 0;                                             \
       const size_t smem_bytes = 1024 + na * a_stage + (res ? wbytes : (size_t)nb * (size_t)p.b_tile_bytes) + SM::tail_bytes(); \
-      auto kern = conv_igemm_kernel<BN_, PAIR_, STACK_>;                                                          \
+      auto kern = conv_igemm_kernel<BN_, PAIR_, STACK_, LIN_>;                                                        \
       /* once per kernel instantiation and device: the attribute call costs microseconds on every eager launch */ \
       static thread_local int attr_dev = -1;                                                                      \
       int cur_dev = 0; cudaGetDevice(&cur_dev);                                                                   \
@@ -941,12 +1084,15 @@ extern "C" int stp3_conv_fwd(const stp3_conv_desc* d, const void* x_hi, const vo
       launched_grid = (int)cfg.gridDim.x;                                                                         \
       STP3_CUDA_OK(cudaLaunchKernelEx(&cfg, kern, tm_hi, tm_lo, tm_w, p));                                        \
     } while (0)
-    if (bn_launch == 64) {
-      if (stack) { if (pair) STP3_LAUNCH_CONV(64, true, true); else STP3_LAUNCH_CONV(64, false, true); }
-      else { if (pair) STP3_LAUNCH_CONV(64, true, false); else STP3_LAUNCH_CONV(64, false, false); }
-    } else {
-      if (pair) STP3_LAUNCH_CONV(128, true, false); else STP3_LAUNCH_CONV(128, false, false);
+#define STP3_DISPATCH_CONV(LIN_)                                                                                  \
+    if (bn_launch == 64) {                                                                                        \
+      if (stack) { if (pair) STP3_LAUNCH_CONV(64, true, true, LIN_); else STP3_LAUNCH_CONV(64, false, true, LIN_); } \
+      else { if (pair) STP3_LAUNCH_CONV(64, true, false, LIN_); else STP3_LAUNCH_CONV(64, false, false, LIN_); }  \
+    } else {                                                                                                      \
+      if (pair) STP3_LAUNCH_CONV(128, true, false, LIN_); else STP3_LAUNCH_CONV(128, false, false, LIN_);         \
     }
+    if (linear) { STP3_DISPATCH_CONV(true) } else { STP3_DISPATCH_CONV(false) }
+#undef STP3_DISPATCH_CONV
 #undef STP3_LAUNCH_CONV
     STP3_CUDA_OK(cudaGetLastError());
   }

@@ -174,6 +174,26 @@ __device__ __forceinline__ void tma_load_5d_pair(void* dst, const CUtensorMap* m
       : "memory");
 }
 
+// im2col mode (rank-4 (N, H, W, C) tensor map from cuTensorMapEncodeIm2col): pixelsPerColumn consecutive pixels of the
+// map's bounding box, starting at (n, h, w) and walking W, then H, then N, each read at (h + off_h, w + off_w);
+// pixels outside the tensor are zero-filled.  One pixel = one channelsPerPixel-wide shared-memory row.
+__device__ __forceinline__ void tma_load_im2col_4d(void* dst, const CUtensorMap* m, uint64_t* bar, int c, int w, int h,
+                                                   int n, uint16_t off_w, uint16_t off_h) {
+  asm volatile(
+      "cp.async.bulk.tensor.4d.shared::cluster.global.im2col.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], "
+      "[%2], {%7, %8};" ::"r"(smem_u32(dst)),
+      "l"(m), "r"(smem_u32(bar)), "r"(c), "r"(w), "r"(h), "r"(n), "h"(off_w), "h"(off_h)
+      : "memory");
+}
+__device__ __forceinline__ void tma_load_im2col_4d_pair(void* dst, const CUtensorMap* m, uint32_t bar_cluster, int c,
+                                                        int w, int h, int n, uint16_t off_w, uint16_t off_h) {
+  asm volatile(
+      "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.im2col.mbarrier::complete_tx::bytes [%0], [%1, {%3, "
+      "%4, %5, %6}], [%2], {%7, %8};" ::"r"(smem_u32(dst)),
+      "l"(m), "r"(bar_cluster), "r"(c), "r"(w), "r"(h), "r"(n), "h"(off_w), "h"(off_h)
+      : "memory");
+}
+
 // ---------------------------------------------------------------- tcgen05 / TMEM
 template <uint32_t kCols>
 __device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem) {   // one full warp; writes the base address to smem

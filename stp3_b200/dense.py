@@ -139,7 +139,10 @@ def pack_conv(weight: torch.Tensor, bias: torch.Tensor, *, stride: int = 1, dila
 
 # ------------------------------------------------------------------------------------------------ autotuner
 # The conv kernel has two tiling knobs (sub-tiles per CTA tile -- or a 16x16 tile shared by a CTA pair through
-# tcgen05.mma.cta_group::2, n_sub = 3 -- and sharing one activation load between the dy taps of a 3x3).  Which combination wins depends on the layer (K depth, N width, image size, whether the weights are
+# tcgen05.mma.cta_group::2, n_sub = 3 -- and sharing one activation load between the dy taps of a 3x3).  2-D layers over
+# every frame also get the linear tiling (n_sub 4 / 5 = 128 / 256 consecutive output pixels per CTA / CTA pair, one
+# im2col load per tap; no pixels of padding on small maps, and a 256-column layer runs as one launch).  Which
+# combination wins depends on the layer (K depth, N width, image size, whether the weights are
 # smem-resident), so the first eager call of every (layer, shape) times the candidates back to back and the winner is
 # cached; CUDA-graph capture then records the tuned launches.  STP3_CONV_AUTOTUNE=0 disables it (kernel heuristics).
 import os as _os
@@ -150,10 +153,13 @@ _TUNE_PAIR = _os.environ.get("STP3_CONV_PAIR", "1") != "0"
 TUNE_LOG = []      # (description, {config: ms}) for reports
 
 
-def _tune(key, desc, launch, groupable, ntaps=1, bn=0):
+def _tune(key, desc, launch, groupable, ntaps=1, bn=0, linear=False):
     cands = [(1, 1), (2, 1)] + ([(1, 3), (2, 3)] if groupable else [])
     if _TUNE_PAIR:
         cands += [(3, 1)] + ([(3, 3)] if groupable else [])
+    if linear:          # group 3 / 1 only picks the tap order (the same as the 2-D tiling with that group)
+        for ns in ((4, 5) if _TUNE_PAIR else (4,)):
+            cands += [(ns, 1)] + ([(ns, 3)] if groupable else [])
     if ntaps > 1:       # weights streamed through the ring instead of resident: more activation stages in flight
         cands += [(ns, g + 4) for ns, g in cands if ns != 1]
     if bn == 64:        # stacked [W_hi; W_lo] operand: two MMAs per product instead of three
@@ -186,8 +192,8 @@ def conv(x: HL, pc: PackedConv, *, cin_off: int = 0, out: Optional[HL] = None, o
     out2 (bn = 128 layers, n_store <= 64): output columns [64, 64+n_store2) go to out2[..., out2_coff:...] with activation
     relu2 -- two 64-column convolutions of the same input in one launch.
     col_sums (B*T, 64) fp32 (bn = 64 layers): receives the per-image sums over pixels of the activated output.
-    tune = (n_sub, group) forces a tiling (n_sub 3 = CTA pair; group +4 = streamed weights, +8 = stacked hi/lo weight
-    operand) instead of the autotuned one."""
+    tune = (n_sub, group) forces a tiling (n_sub 3 = CTA pair, 4 / 5 = linear tiling per CTA / CTA pair; group +4 =
+    streamed weights, +8 = stacked hi/lo weight operand) instead of the autotuned one."""
     B, T_total, H, W, cs = x.hi.shape
     t0, T = frames if frames is not None else (0, T_total)      # process frames [t0, t0+T) of every sample
     Ho, Wo = out_hw if out_hw is not None else ((H + pc.stride - 1) // pc.stride, (W + pc.stride - 1) // pc.stride)
@@ -263,7 +269,9 @@ def conv(x: HL, pc: PackedConv, *, cin_off: int = 0, out: Optional[HL] = None, o
         ins = {x.hi.data_ptr(), x.lo.data_ptr()} | ({residual.hi.data_ptr(), residual.lo.data_ptr()} if residual is not None else set())
         outs = {t.data_ptr() for t in ((out.hi, out.lo) if out is not None else ()) + ((out2.hi, out2.lo) if out2 is not None else ())}
         assert not (ins & outs), "stp3_b200.dense.conv: output aliases an input (in-place convolution is not supported)"
-        cfg = _tune(key, desc, launch, groupable, len(taps), pc.bn)
+        linear = (all(t[0] == 0 for t in taps) and (t0, T) == (0, T_total) and col_sums is None and hd is None and
+                  img_bias is None and out_f32 is None)
+        cfg = _tune(key, desc, launch, groupable, len(taps), pc.bn, linear)
     launch(*(cfg or (0, 0)))
     return out
 
